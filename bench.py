@@ -21,6 +21,10 @@ Output: ONE JSON line on rank 0.
     python bench.py --workload m               # config M
     torchrun ... bench.py --gpus 8             # one rank per GPU
     python bench.py --impl reference           # CPU arm: the oracle port on all host cores
+    python bench.py --dump-outputs DIR         # also write the last timed step's outputs as DIR/<name>.npy
+
+The bench runs the native libraries that ``__graft_entry__.build()`` left in the tree and writes nothing into the tree,
+so it also runs from a read-only checkout.
 """
 from __future__ import annotations
 
@@ -36,6 +40,7 @@ from pathlib import Path
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # no __pycache__ next to the package sources
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
@@ -224,8 +229,6 @@ def cpu_pass_setup(workload: str, sample_rows: int, ncols: int):
     (parallel first touch: every page lives on the NUMA node of the thread that reads it), returns one_pass()."""
     os.environ.setdefault("OMP_PROC_BIND", "close")
     os.environ.setdefault("OMP_PLACES", "cores")
-    from learningorchestra_b200.build import build_oracle
-    build_oracle()
     import ctypes as C
     from oracle import cport
     threads = cport.use_all_cores()
@@ -461,13 +464,46 @@ def load_goldens(workload: str, rows: int, ncols: int):
     return g
 
 
+DUMP_SAMPLE_BYTES = 32 << 20      # --dump-outputs: size of the sample of the fp32 output table
+
+
+def dump_outputs(dump_dir: str, sh, out, k: int, nbins: int) -> list[Path]:
+    """Writes what the last step handed its caller, as ``dump_dir/<name>.npy``, so that two builds can be compared
+    output for output on identical inputs:
+
+    * ``counts``: the merged ``k x nbins`` histogram, float64 (exact: every count is below 2^53);
+    * ``out_f32_sample``: ``k x S`` float32, the same S rows of every projected output column, drawn without replacement
+      by a generator seeded with SEED and kept in row order; S is what fits in DUMP_SAMPLE_BYTES.  The rows come from
+      this rank's shard, which is the whole table on one GPU.
+    """
+    import torch
+    arrays = {}
+    if nbins:
+        arrays["counts"] = sh.result(k * nbins).reshape(k, nbins).astype(np.float64)
+    if out is not None:
+        shard = out.shards[0]
+        n = min(shard.nrows, DUMP_SAMPLE_BYTES // (4 * k))
+        rows = torch.from_numpy(np.sort(np.random.default_rng(SEED).choice(shard.nrows, size=n, replace=False))).cuda()
+        cols = [torch.as_tensor(shard.column_view(j), device="cuda")[rows] for j in range(k)]
+        arrays["out_f32_sample"] = torch.stack(cols).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 * 10 ** 6:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed 64 MB")
+    d = Path(dump_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    paths = []
+    for name, a in arrays.items():
+        paths.append(d / f"{name}.npy")
+        np.save(paths[-1], a)
+    return paths
+
+
 def run_gpu(args) -> int:
     real_stdout = _claim_stdout()
     import torch
     import torch.distributed as dist
 
     from learningorchestra_b200 import _native as N
-    from learningorchestra_b200.build import build_native
     from learningorchestra_b200.engine import Engine
     from learningorchestra_b200.sharding import ShardedEngine
 
@@ -481,10 +517,6 @@ def run_gpu(args) -> int:
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    if rank == 0:
-        build_native()                      # no-op when the in-tree .so is newer than its sources
-    if world > 1:
-        dist.barrier()                      # nobody loads libloexec.so while rank 0 might be rewriting it
 
     w = args.workload
     eng = Engine(local_rank)
@@ -561,6 +593,12 @@ def run_gpu(args) -> int:
     torch.cuda.synchronize()
     sampler.mark_end()
     launches = eng.launch_count - launches0 - 1          # the barrier launch is outside the timed region
+    if args.dump_outputs:
+        if rank == 0:
+            for p in dump_outputs(args.dump_outputs, sh, out, k, NBINS if w != "s10" else 0):
+                log(f"wrote {p}")
+        if world > 1:
+            dist.barrier()                               # the merge of the next step waits for rank 0
     for _ in range(5):                                   # the same step in isolation (event-bracketed, serialised)
         step(True)
     torch.cuda.synchronize()
@@ -774,7 +812,13 @@ def main():
                     help="serialise consecutive steps completely (no programmatic dependent launch between them)")
     ap.add_argument("--merge", default="auto", choices=["auto", "nccl", "p2p", "peer"],
                     help="N > 1: how partial histograms are merged (in-kernel peer-memory merge, or NCCL all-reduce)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none to write")
     args.rows = args.rows or WORKLOADS[args.workload]["rows"]
     args.cols = args.cols or WORKLOADS[args.workload]["cols"]
     global K_SELECT

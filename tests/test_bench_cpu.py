@@ -26,3 +26,8 @@ def test_reference_arm_other_ranks_exit_quietly(built):
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--gpus", "8", "--steps", "1",
                           "--warmup", "0"], capture_output=True, text=True, timeout=120, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr

@@ -408,3 +408,32 @@ def test_more_projected_columns_than_one_launch_holds(engine):
     got8 = engine.hist_u8_cols(t8, idx).to_numpy()
     np.testing.assert_array_equal(got8, bn.hist_u8_cols(tb, idx))
     t8.free()
+
+
+def test_bench_dumps_the_last_timed_steps_outputs(built, tmp_path):
+    """``bench.py --dump-outputs``: the merged counts and the sampled fp32 output rows of the last timed step equal the
+    oracle's, and ``--steps`` is the number of timed launches."""
+    import json
+    import subprocess
+    import sys
+    from pathlib import Path
+    rows, ncols = 300_007, 32
+    bench = Path(__file__).resolve().parent.parent / "bench.py"
+    res = subprocess.run([sys.executable, str(bench), "--rows", str(rows), "--steps", "7", "--warmup", "1", "--no-e2e",
+                          "--no-cpu", "--executor-rows", "0", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stderr[-3000:]
+    line = json.loads(res.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 7 and line["gpu_launches"] == 7
+    counts = np.load(tmp_path / "counts.npy")
+    sample = np.load(tmp_path / "out_f32_sample.npy")
+    assert counts.dtype == np.float64 and sample.dtype == np.float32 and sample.shape[0] == ncols
+    assert counts.nbytes + sample.nbytes <= 64 * 10 ** 6
+    cols = [(7 * j + 3) % ncols for j in range(ncols)]
+    lo, hi = np.full(ncols, -1000.0, np.float32), np.full(ncols, 1000.0, np.float32)
+    exp_counts, _ = cport.synth_project_cast_hist(0, SEED, 0, rows, -1000.0, 1000.0, cols, 256, lo, hi)
+    np.testing.assert_array_equal(counts, exp_counts.astype(np.float64))
+    picked = np.sort(np.random.default_rng(SEED).choice(rows, size=sample.shape[1], replace=False))
+    for j, c in enumerate(cols):
+        exp = cport.cast_f64_f32(cport.synth_f64(0, SEED, c, 0, rows))[picked]
+        np.testing.assert_array_equal(_bits(sample[j]), _bits(exp))
